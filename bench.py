@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # ours (torchrun launches N ranks for N > 1)
     python bench.py --impl reference --gpus N ...            # unmodified reference from baseline/_ref
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 Metric (BASELINE.json): training tokens/s for the WHOLE job, device-timed with CUDA events, max over ranks.
 Weak scaling: the per-GPU batch is fixed (``--mbs``, default 2 sequences of 4096 tokens).
@@ -50,7 +51,15 @@ def parse():
     p.add_argument("--trace", default=None, help="write a kernel timeline (chrome trace) of one extra, untimed step")
     p.add_argument("--no-comm-trace", action="store_true",
                    help="skip the extra profiled step that measures exposed communication when N > 1")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", default=None, metavar="DIR",
+                   help="ours: after the timed steps write what the last one computed as DIR/<name>.npy (loss, "
+                        "gradient norm, a fixed sample of the updated weights) to compare two builds output for output")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs is only implemented for --impl ours")
+    return a
 
 
 class ClockSampler:
@@ -96,6 +105,40 @@ def bench_config(a, world, layers):
 
 
 METRIC = "Llama-3-8B FSDP bf16 training throughput (whole job, device-timed, max over ranks)"
+
+PARAM_SAMPLE = 8192     # positions per parameter in --dump-outputs: 1.33M fp32 values (5.3 MB) for Llama-3-8B
+
+
+def dump_outputs(out_dir, model, last, rank, world):
+    """Write what the last timed step computed: its loss, its gradient norm before clipping and the updated fp32
+    master weights -- of every parameter all of it, or PARAM_SAMPLE seeded positions when it is larger.  Parameters
+    are taken in the order of their names, so the sample does not depend on how the engine groups them into flat
+    shards; each rank contributes the positions it owns and a sum over ranks assembles the whole sample."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    from torchacc_b200.parallel.state_dict_utils import get_shard_metadata
+    meta = get_shard_metadata(model.engine)
+    params = sorted(((um["prefix"] + "." if um["prefix"] else "") + p["fqn"], p, um["shard_numel"], shard)
+                    for um, shard in zip(meta["units"], model.parameters()) for p in um["params"])
+    g = torch.Generator().manual_seed(0)
+    parts = []
+    with torch.no_grad():
+        for _, p, shard_numel, shard in params:
+            n = p["numel"]
+            idx = torch.arange(n) if n <= PARAM_SAMPLE else \
+                torch.randint(0, n, (PARAM_SAMPLE,), generator=g).sort().values
+            pos = (p["offset"] - meta["rank"] * shard_numel + idx).to(shard.device)
+            own = (pos >= 0) & (pos < shard_numel)
+            parts.append(torch.where(own, shard[pos.clamp(0, shard_numel - 1)], 0.0))
+        weights = torch.cat(parts)
+        if world > 1:
+            dist.all_reduce(weights)
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        outs = {"loss": last["loss"], "grad_norm": last["grad_norm"], "weights_sample": weights}
+        for name, t in outs.items():
+            np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def hf_llama(a, torch, device, world):
@@ -212,7 +255,7 @@ def run_ours(a):
         out = model(**batch)
         loss = out["loss"]
         loss.backward()
-        model.clip_grad_norm_(1.0)
+        last["grad_norm"] = model.clip_grad_norm_(1.0)
         opt.step()
         model.zero_grad()
         last["loss"] = loss
@@ -231,6 +274,8 @@ def run_ours(a):
     clocks = sampler.stop() if sampler else None
     tokens = a.mbs * a.seq_len * world * a.steps
     value = tokens / (ms / 1e3)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, model, last, rank, world)     # before any further step changes the weights
 
     # ---- end-to-end through the public API: AsyncLoader H2D every step + loss D2H every step ---------------------
     e2e = None

@@ -91,6 +91,35 @@ def test_grad_accumulation_matches_single_batch(grad_dtype, tol):
     assert rel < tol, float(rel)
 
 
+def test_bench_dump_outputs_is_reproducible(tmp_path):
+    """bench.py --dump-outputs: the last timed step's loss, gradient norm and weight sample come out as float32 .npy
+    files within 64 MB, and a second run with the same arguments computes the same thing."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+    def run(d):
+        cmd = [sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+               "--layers", "1", "--seq-len", "512", "--mbs", "1", "--no-e2e", "--dump-outputs", str(d)]
+        p = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+        assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-3000:]
+        res = json.loads([l for l in p.stdout.splitlines() if l.startswith("{")][-1])
+        assert res["steps"] == 2 and res["warmup"] == 1
+        return {f[:-4]: np.load(d / f) for f in sorted(os.listdir(d))}
+
+    a, b = run(tmp_path / "a"), run(tmp_path / "b")
+    assert sorted(a) == ["grad_norm", "loss", "weights_sample"]
+    assert all(v.dtype == np.float32 and np.isfinite(v).all() for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    np.testing.assert_allclose(a["loss"], b["loss"], rtol=1e-3)
+    np.testing.assert_allclose(a["grad_norm"], b["grad_norm"], rtol=1e-2)
+    # three AdamW steps at lr 1e-5 move a weight by at most a few 1e-5, whatever the order of the float sums
+    np.testing.assert_allclose(a["weights_sample"], b["weights_sample"], rtol=0, atol=1e-4)
+
+
 def test_hf_llama_through_accelerate_uses_native_attention_and_rope():
     """accelerate(HF LlamaForCausalLM): linears, RMSNorm, SwiGLU, RoPE, attention and the loss run on the native kernels
     (round-1 review: the HF path fell back to the flash-attn library and HF's elementwise RoPE) and the loss / its

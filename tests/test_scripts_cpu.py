@@ -47,19 +47,19 @@ def test_example_train_llama_fsdp_single_process(tmp_path):
     assert any(f.endswith(".pth") for f in os.listdir(tmp_path / "ck")), os.listdir(tmp_path / "ck")
 
 
-def test_accuracy_benchmark_tiny():
+def test_accuracy_benchmark_tiny(tmp_path):
     out = _run(["bash", "benchmarks/accuracy/run.sh"],
-               env={"MODEL": "tiny", "LAYERS": "2", "STEPS": "12", "SEQ": "64", "BS": "2", "OUT": "/tmp/tb_acc_test"})
+               env={"MODEL": "tiny", "LAYERS": "2", "STEPS": "12", "SEQ": "64", "BS": "2", "OUT": str(tmp_path)})
     res = json.loads(out.strip().splitlines()[-1])
     assert res["pass"] and res["abs_delta"] <= 1e-2
 
 
-def test_accuracy_benchmark_tiny_hf_model():
+def test_accuracy_benchmark_tiny_hf_model(tmp_path):
     """Same protocol on the HuggingFace LlamaForCausalLM object (kernel patches + fused linear-CE through accelerate())."""
     pytest.importorskip("transformers")
     out = _run(["bash", "benchmarks/accuracy/run.sh"],
                env={"MODEL": "tiny", "LAYERS": "2", "STEPS": "12", "SEQ": "64", "BS": "2", "HF": "1",
-                    "OUT": "/tmp/tb_acc_test_hf"})
+                    "OUT": str(tmp_path)})
     res = json.loads(out.strip().splitlines()[-1])
     assert res["pass"] and res["abs_delta"] <= 1e-2
 
